@@ -365,6 +365,28 @@ def parity_check(a, ctx, ix, base, d, rd, nsample):
             "reference": "oracle/_ref/centrifuge-class -p %d --reorder, same index, same FASTQ (%.1f s)" % (p, t_ref)}
 
 
+DUMP_UNITS = 1 << 17
+
+
+def dump_outputs(out_dir, ctx, first, taxids, counts):
+    """The last timed step's outputs, as a caller of the resident path receives them: the step's per-taxon counters
+    (cfb_counts_dense after the all-reduce) and the records of its last window (cfb_resident_result holds that window
+    only), of which a fixed sample of units is kept.  float64 holds every value exactly (counts and taxIDs < 2^53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    off, recs = ctx.resident_result()
+    off = off.astype(np.int64)
+    n = len(off) - 1
+    units = np.sort(np.random.default_rng(20240601).choice(n, min(n, DUMP_UNITS), replace=False))
+    cnt = off[units + 1] - off[units]
+    idx = np.repeat(off[units], cnt) + np.arange(int(cnt.sum())) - np.repeat(np.cumsum(cnt) - cnt, cnt)
+    out = {"counts_taxid": taxids, "counts": counts, "sample_unit": first + units, "sample_records_per_unit": cnt}
+    for f in ("taxid", "score", "hitlen", "uid"):
+        out["sample_record_" + f] = recs[f][idx]
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+    log("outputs of the last timed step written to %s (%s)" % (out_dir, ", ".join(sorted(out))))
+
+
 def measured_peak():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -406,6 +428,8 @@ def parse_args():
     ap.add_argument("--cpu-sample", type=int, default=int(os.environ.get("CFB_BENCH_CPU_SAMPLE", 400000)))
     ap.add_argument("--parity-reads", type=int, default=int(os.environ.get("CFB_BENCH_PARITY_READS", 200000)), help="units of the step batch checked against the reference binary (un-timed)")
     ap.add_argument("--skip-arms", default=os.environ.get("CFB_BENCH_SKIP", ""), help="comma list of e2e_byteform,e2e_text,cpu_baseline,gather to leave out (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64): "
+                    "its all-reduced per-taxon counters, and the records of a fixed, seeded sample of %d units of its last window" % DUMP_UNITS)
     a = ap.parse_args()
     if a.genera == 0:
         a.genera = max(1, int(round(a.index_gbp * 1e9 / (a.species * a.genome_len))))
@@ -615,6 +639,8 @@ def _main(result):
                     "unique_units_global": int(step_counts[1].sum()), "units_global": int(world * n),
                     "equals_sum_of_local_vectors": bool(np.array_equal(local_counts.cpu().numpy().astype(np.uint64), step_counts))}
     kms_step = kms / a.steps
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, ctx, windows[-1][0], ctx.counts_taxids()[:n_tax], step_counts)
 
     # ---------------- e2e arms: host buffers in, host results out, sub-batches streaming over the context's slots
     nslots = min(ctx.n_slots, E2E_SLOTS)

@@ -4,12 +4,9 @@ random option sets.
   * the oracle's file driver against the unmodified reference binary: classification TSV and report, byte for byte;
   * the product's per-thread logic (cf_logic.h compiled for the host, the code the CUDA kernels run) against the
     oracle, record by record."""
-import os
 import random
-import subprocess
 
 import numpy as np
-import pytest
 
 import util
 from util_fuzz import clean_reads
@@ -51,7 +48,6 @@ API_OPTS = [dict(), dict(k=1), dict(k=3), dict(k=50), dict(min_hitlen=15), dict(
             dict(min_hitlen=16, k=1, rank_slot=2)]
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
 def test_oracle_matches_reference_on_random_reads_and_options(tmp_path):
     util.ensure_oracle()
     base = util.golden_index("adv")
@@ -71,9 +67,9 @@ def test_oracle_matches_reference_on_random_reads_and_options(tmp_path):
             args += ["-U", p1]
         with open(p1, "wb") as f:
             f.write(fa(rs))
-        a = util.run_cli(util.REF_CLASS, args, str(tmp_path / "r.tsv"), str(tmp_path / "r.rep"))
+        a = util.reference_cli(args, tmp_path)
         b = util.run_cli(util.ORACLE_BIN, args, str(tmp_path / "o.tsv"), str(tmp_path / "o.rep"))
-        assert a == b, (case, opts, paired)
+        assert a == util.digests(b), (case, opts, paired)
 
 
 def test_product_logic_matches_oracle_on_random_reads_and_options():

@@ -114,18 +114,14 @@ def test_bench_configuration_all_tables_matches_oracle_and_reference(tmp_path):
     ix = m.Index(base, -1)
     assert ix.info.compressed == 1 and ix.info.len > (1 << 32)
     ix.close()
-    if not util.have_ref():
-        pytest.skip("oracle/_ref reference binaries not shipped")
     fq = str(tmp_path / "r.fq")
     write_fastq(fq, codes)
-    ref = util.run_cli(util.REF_CLASS, ["-q", "-x", base, "-U", fq, "-p", "16", "--reorder"], str(tmp_path / "a.tsv"), str(tmp_path / "a.rep"))
+    ref = util.reference_cli(["-q", "-x", base, "-U", fq, "-p", "16", "--reorder"], tmp_path)
     env = dict(os.environ, CFB_FULL_TABLES="1")
     subprocess.check_call([EXE, "-q", "-x", base, "-U", fq, "-S", str(tmp_path / "b.tsv"), "--report-file", str(tmp_path / "b.rep")],
                           env=env, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    with open(tmp_path / "b.tsv", "rb") as f:
-        assert f.read() == ref[0]
-    with open(tmp_path / "b.rep", "rb") as f:
-        assert f.read() == ref[1]
+    assert util.file_digest(tmp_path / "b.tsv") == ref[0]
+    assert util.file_digest(tmp_path / "b.rep") == ref[1]
 
 
 @BIG

@@ -1,13 +1,12 @@
 """GPU suite for the index builder: cfb_build_index must write the bytes centrifuge-build-bin writes."""
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import util
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not util.have_ref(), reason="needs oracle/_ref/centrifuge-build-bin as the checker")]
+pytestmark = pytest.mark.gpu
 
 
 def capi():
@@ -15,28 +14,28 @@ def capi():
     return m
 
 
-def ref_build(fa, conv, nodes, names, base, extra=()):
-    subprocess.check_call([util.REF_BUILD, "-p", "4", "--conversion-table", conv, "--taxonomy-tree", nodes, "--name-table", names]
-                          + list(extra) + [fa, base], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+def ref_build(fa, conv, nodes, names, base):
+    """digests of the .1-.4.cf files centrifuge-build-bin writes (recorded reference run)"""
+    r = util.reference_run("build", ["-p", "4", "--conversion-table", conv, "--taxonomy-tree", nodes, "--name-table", names, fa], base)
+    assert r["rc"] == 0, r
+    return r["outputs"]
 
 
-def assert_same_index(a, b):
-    for k in "1234":
-        with open("%s.%s.cf" % (a, k), "rb") as f, open("%s.%s.cf" % (b, k), "rb") as g:
-            x, y = f.read(), g.read()
-        if x != y:
-            n = min(len(x), len(y))
-            d = next((i for i in range(n) if x[i] != y[i]), n)
-            raise AssertionError(".%s.cf differs: sizes %d vs %d, first difference at byte %d" % (k, len(x), len(y), d))
+def assert_same_index(want, b):
+    """`want`: digests of the reference's .1-.4.cf files.  To see where a file differs, record the run again
+    (CFB_RECORD_REFERENCE, tests/util.py): the reference's files are then written beside the product's."""
+    for k, w in zip("1234", want):
+        f = "%s.%s.cf" % (b, k)
+        assert util.file_digest(f) == w, ".%s.cf (%d bytes) differs from the reference's" % (k, os.path.getsize(f))
 
 
 def test_builder_matches_reference_adversarial(tmp_path):
     m = capi()
     d = str(tmp_path)
     util.synth.write_adversarial(d, seed=33, n_reads=10)
-    ref_build(d + "/genomes.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
+    want = ref_build(d + "/genomes.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
     m.build_index(m.build_opts(d + "/mine", fasta=[d + "/genomes.fa"], conversion_table=d + "/conv.tsv", taxonomy_tree=d + "/nodes.dmp", name_table=d + "/names.dmp"))
-    assert_same_index(d + "/ref", d + "/mine")
+    assert_same_index(want, d + "/mine")
 
 
 def test_builder_matches_reference_gaps_descriptions_multifile(tmp_path):
@@ -64,9 +63,9 @@ def test_builder_matches_reference_gaps_descriptions_multifile(tmp_path):
             f.write("%d\t|\t100\t|\tspecies\t|\n" % (1000 + t))
     with open(d + "/names.dmp", "w") as f:
         f.write("1\t|\troot\t|\t\t|\tscientific name\t|\n100\t|\tSome genus\t|\t\t|\tscientific name\t|\n1001\t|\tSp one two\t|\t\t|\tscientific name\t|\n")
-    ref_build(d + "/a.fa," + d + "/b.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
+    want = ref_build(d + "/a.fa," + d + "/b.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
     m.build_index(m.build_opts(d + "/mine", fasta=[d + "/a.fa", d + "/b.fa"], conversion_table=d + "/conv.tsv", taxonomy_tree=d + "/nodes.dmp", name_table=d + "/names.dmp"))
-    assert_same_index(d + "/ref", d + "/mine")
+    assert_same_index(want, d + "/mine")
 
 
 def test_builder_synthetic_mode_matches_reference(tmp_path):
@@ -76,9 +75,9 @@ def test_builder_synthetic_mode_matches_reference(tmp_path):
     conv, nodes, names = m.write_synth_taxonomy(d, 4, 5, 30000)
     o = m.build_opts(d + "/mine", synth=(4, 5, 30000, 77, 0.03), conversion_table=conv, taxonomy_tree=nodes, name_table=names)
     m.synth_fasta(o, d + "/g.fa")
-    ref_build(d + "/g.fa", conv, nodes, names, d + "/ref")
+    want = ref_build(d + "/g.fa", conv, nodes, names, d + "/ref")
     m.build_index(o)
-    assert_same_index(d + "/ref", d + "/mine")
+    assert_same_index(want, d + "/mine")
     # reads sampled from the same generator classify to their source species
     codes = m.synth_reads(o, 2000, 100, 5)
     assert codes.shape == (2000, 100) and codes.max() <= 4
@@ -103,9 +102,9 @@ def test_builder_many_sequences_wide_sample(tmp_path):
             f.write("%d\t|\t1\t|\tspecies\t|\n" % (1000 + t))
     with open(d + "/names.dmp", "w") as f:
         f.write("1\t|\troot\t|\t\t|\tscientific name\t|\n")
-    ref_build(d + "/g.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
+    want = ref_build(d + "/g.fa", d + "/conv.tsv", d + "/nodes.dmp", d + "/names.dmp", d + "/ref")
     m.build_index(m.build_opts(d + "/mine", fasta=[d + "/g.fa"], conversion_table=d + "/conv.tsv", taxonomy_tree=d + "/nodes.dmp", name_table=d + "/names.dmp"))
-    assert_same_index(d + "/ref", d + "/mine")
+    assert_same_index(want, d + "/mine")
 
 
 def test_bench_data_path_matches_reference_end_to_end(tmp_path):
@@ -129,9 +128,9 @@ def test_bench_data_path_matches_reference_end_to_end(tmp_path):
         files = [d + "/%s_%d.fq" % (tag, k + 1) for k in range(rd.mates)]
         bench.write_fastq_files(rd, files)
         rargs = ["-q", "-x", d + "/idx"] + (["-1", files[0], "-2", files[1]] if paired else ["-U", files[0]])
-        a = util.run_cli(util.REF_CLASS, rargs, d + "/a.tsv", d + "/a.rep")
+        a = util.reference_cli(rargs, tmp_path)
         b = util.run_cli(exe, rargs + ["--batch-units", "7000"], d + "/b.tsv", d + "/b.rep")
-        assert a[0] == b[0], tag
-        assert a[1] == b[1], tag
-        rows = a[0].decode().strip().split("\n")[1:]
+        assert a[0] == util.digest(b[0]), tag
+        assert a[1] == util.digest(b[1]), tag
+        rows = b[0].decode().strip().split("\n")[1:]
         assert sum(1 for r in rows if "unclassified" not in r) > 15000, tag      # the synthetic reads do classify

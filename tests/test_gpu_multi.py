@@ -25,14 +25,6 @@ def n_devices():
     return int(capi().lib().cfb_device_count())
 
 
-def first_diff(a, b):
-    la, lb = a.split(b"\n"), b.split(b"\n")
-    for i, (x, y) in enumerate(zip(la, lb)):
-        if x != y:
-            return "line %d: ours %r / reference %r (lines %d / %d)" % (i, x, y, len(la), len(lb))
-    return "lengths %d / %d" % (len(la), len(lb))
-
-
 def fastq_bytes(reads):
     return b"".join(b"@" + n.encode() + b"\n" + a.tobytes() + b"\n+\n" + b"I" * len(a) + b"\n" for n, a in reads)
 
@@ -102,7 +94,6 @@ def test_allreduce_on_a_communicator_of_one(syn):
     ctx.close(); c2.close(); ix.close()
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
 def test_read_files_are_separate_pattern_sources(syn, tmp_path):
     """Centrifuge runs its inputs one file (pair) at a time (centrifuge.cpp:3006-3046): unnamed reads of a second -U file
     are numbered from 0 again, the report covers all files, and -1/-2 lists must match file by file."""
@@ -115,10 +106,9 @@ def test_read_files_are_separate_pattern_sources(syn, tmp_path):
         f.write(b"".join(b"@\n" + a.tobytes() + b"\n+\n" + b"I" * len(a) + b"\n" for _, a in rd[500:]))
     for extra in ([], ["--host-parse"]):
         args = ["-q", "-x", base, "-U", fa + "," + fb] + extra
-        want = util.run_cli(util.REF_CLASS, args[:5], str(tmp_path / "r.tsv"), str(tmp_path / "r.rep"))
+        want = util.reference_cli(args[:5], tmp_path)
         got = util.run_cli(EXE, args, str(tmp_path / "o.tsv"), str(tmp_path / "o.rep"))
-        assert got[0] == want[0], first_diff(got[0], want[0])
-        assert got[1] == want[1], first_diff(got[1], want[1])
+        assert util.digests(got) == want, extra
     m1 = [(n, a) for n, a in rd[:600]]; m2 = [(n, a[::-1].copy()) for n, a in rd[:600]]
     paths = {}
     for tag, lst, cut in (("a", m1, 250), ("b", m2, 400)):      # the -1 list is cut after 250 records, the -2 list after 400
@@ -127,9 +117,10 @@ def test_read_files_are_separate_pattern_sources(syn, tmp_path):
             with open(paths[tag, k], "wb") as f:
                 f.write(fastq_bytes(part))
     args = ["-q", "-x", base, "-1", paths["a", 0] + "," + paths["a", 1], "-2", paths["b", 0] + "," + paths["b", 1]]
-    for exe in (util.REF_CLASS, EXE):
-        p = subprocess.run([exe] + args + ["-S", str(tmp_path / "x.tsv"), "--report-file", str(tmp_path / "x.rep")], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
-        assert p.returncode != 0 and b"fewer reads in file specified with -1" in p.stderr
+    r = util.reference_run("class", args, str(tmp_path / "ref"))
+    assert r["rc"] != 0 and any("fewer reads in file specified with -1" in l for l in r["errors"]), r
+    p = subprocess.run([EXE] + args + ["-S", str(tmp_path / "x.tsv"), "--report-file", str(tmp_path / "x.rep")], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+    assert p.returncode != 0 and b"fewer reads in file specified with -1" in p.stderr
     # equal cuts: two file pairs, one after the other
     for tag, lst in (("c", m1), ("d", m2)):
         for k, part in enumerate((lst[:300], lst[300:])):
@@ -137,10 +128,9 @@ def test_read_files_are_separate_pattern_sources(syn, tmp_path):
             with open(paths[tag, k], "wb") as f:
                 f.write(fastq_bytes(part))
     args = ["-q", "-x", base, "-1", paths["c", 0] + "," + paths["c", 1], "-2", paths["d", 0] + "," + paths["d", 1], "-U", fb]
-    want = util.run_cli(util.REF_CLASS, args, str(tmp_path / "r2.tsv"), str(tmp_path / "r2.rep"))
+    want = util.reference_cli(args, tmp_path)
     got = util.run_cli(EXE, args, str(tmp_path / "o2.tsv"), str(tmp_path / "o2.rep"))
-    assert got[0] == want[0], first_diff(got[0], want[0])
-    assert got[1] == want[1], first_diff(got[1], want[1])
+    assert util.digests(got) == want
 
 
 @pytest.mark.skipif(n_devices() < 2, reason="needs two GPUs (gpurun --gpus 2)")
@@ -161,9 +151,7 @@ def test_two_gpu_cli_output_is_byte_identical_to_one_gpu(syn, tmp_path):
             assert b"devices, per-taxon counters reduced with NCCL" in p.stderr
         outs.append(tuple(open(str(tmp_path / (tag + ext)), "rb").read() for ext in (".tsv", ".rep", ".kr")))
     assert outs[0] == outs[1] == outs[2]
-    if util.have_ref():
-        want = util.run_cli(util.REF_CLASS, ["-q", "-x", base, "-U", fq], str(tmp_path / "ref.tsv"), str(tmp_path / "ref.rep"))
-        assert outs[1][:2] == want
+    assert util.digests(outs[1][:2]) == util.reference_cli(["-q", "-x", base, "-U", fq], tmp_path)
 
 
 @pytest.mark.skipif(n_devices() < 2, reason="needs two GPUs (gpurun --gpus 2)")

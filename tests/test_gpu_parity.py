@@ -234,7 +234,6 @@ def test_cli_tsv_and_report_match_reference_golden(case, adv_base, adv_reads, tm
         assert rep == f.read()
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
 def test_cli_matches_live_reference_paired_fastq(tmp_path):
     base = util.build_index("syn_a", 5, 4, 60000, seed=7, strains=True)
     seqs = util.synth.make_genomes(5, 4, 60000, 7)
@@ -243,9 +242,9 @@ def test_cli_matches_live_reference_paired_fastq(tmp_path):
     util.synth.write_fastq(f1, [(n, x) for n, x, _ in prs])
     util.synth.write_fastq(f2, [(n, y) for n, _, y in prs], qual=b"5")
     exe = os.path.join(util.ROOT, "centrifuge_b200", "centrifuge-class")
-    a = util.run_cli(util.REF_CLASS, ["-q", "-x", base, "-1", f1, "-2", f2], str(tmp_path / "a.tsv"), str(tmp_path / "a.rep"))
+    a = util.reference_cli(["-q", "-x", base, "-1", f1, "-2", f2], tmp_path)
     b = util.run_cli(exe, ["-q", "-x", base, "-1", f1, "-2", f2, "--batch-units", "1000"], str(tmp_path / "b.tsv"), str(tmp_path / "b.rep"))
-    assert a == b
+    assert a == util.digests(b)
 
 
 def test_large_batch_properties():

@@ -1,7 +1,7 @@
 """Text-level operator (SURVEY.md 8f rank 1): FASTQ/FASTA bytes -> TSV on the device.
 
-Every case runs the unmodified reference binary (oracle/_ref) and the drop-in `centrifuge-class` on the
-same files and demands identical classification TSV and report bytes, and checks through the
+Every case runs the drop-in `centrifuge-class` on the files the unmodified reference binary was run on
+(recorded runs, tests/golden/reference_runs.json) and demands identical classification TSV and report bytes, and checks through the
 CFB_TEXT_STATS line which reader handled the input: well-formed files must go through the device
 tokeniser/formatter entirely, files with irregular layout must switch to the record-level reader
 at the span that failed (and still produce the reference's bytes)."""
@@ -14,7 +14,7 @@ import pytest
 
 import util
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")]
+pytestmark = pytest.mark.gpu
 
 EXE = os.path.join(util.ROOT, "centrifuge_b200", "centrifuge-class")
 
@@ -29,15 +29,11 @@ def run_ours(args, tmp, tag, block=None, extra_env=None):
     assert p.returncode == 0, p.stderr.decode()
     m = re.search(r"text operator: (\d+) units in (\d+) spans .* (\d+) fallbacks\); record-level reader: (\d+) units", p.stderr.decode())
     assert m, p.stderr.decode()
-    with open(tsv, "rb") as f:
-        a = f.read()
-    with open(rep, "rb") as f:
-        b = f.read()
-    return (a, b), dict(text=int(m.group(1)), spans=int(m.group(2)), fallbacks=int(m.group(3)), host=int(m.group(4)))
+    return (util.file_digest(tsv), util.file_digest(rep)), dict(text=int(m.group(1)), spans=int(m.group(2)), fallbacks=int(m.group(3)), host=int(m.group(4)))
 
 
 def run_ref(args, tmp, tag):
-    return util.run_cli(util.REF_CLASS, args, str(tmp / (tag + ".tsv")), str(tmp / (tag + ".rep")))
+    return util.reference_cli(args, tmp / tag)
 
 
 @pytest.fixture(scope="module")
@@ -174,13 +170,12 @@ def test_quality_string_errors_match_the_reference(kind, syn, tmp_path):
             if i == 900:
                 q = {"too_many": q + b"FF", "too_few": q[:-1], "space": q[:10] + b" " + q[11:], "control": q[:10] + b"\x1f" + q[11:]}[kind]
             f.write(b"@" + name.encode() + b"\n" + a.tobytes() + b"\n+\n" + q + b"\n")
-    msgs = []
-    for exe in (util.REF_CLASS, EXE):
-        p = subprocess.run([exe, "-q", "-x", base, "-U", fq, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
-                           stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, env=dict(os.environ, CFB_TEXT_BLOCK="30000"))
-        assert p.returncode != 0
-        msgs.append([l for l in p.stderr.decode().splitlines() if l.startswith("Error") or l.startswith("Saw ASCII")])
-    assert msgs[0] and msgs[0] == msgs[1]
+    r = util.reference_run("class", ["-q", "-x", base, "-U", fq], str(tmp_path / "ref"))
+    assert r["rc"] != 0
+    p = subprocess.run([EXE, "-q", "-x", base, "-U", fq, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
+                       stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, env=dict(os.environ, CFB_TEXT_BLOCK="30000"))
+    assert p.returncode != 0
+    assert r["errors"] and r["errors"] == util.error_lines(p.stderr)
 
 
 def test_mate_files_out_of_step_report_the_reference_error(syn, tmp_path):
@@ -189,11 +184,12 @@ def test_mate_files_out_of_step_report_the_reference_error(syn, tmp_path):
     prs = util.synth.sample_pairs(seqs, 800, 100, seed=3)
     f1, f2 = str(tmp_path / "a_1.fq"), str(tmp_path / "a_2.fq")
     write_fq(f1, [(n, x) for n, x, _ in prs], rng); write_fq(f2, [(n, y) for n, _, y in prs][:700], rng)
-    for exe in (util.REF_CLASS, EXE):
-        p = subprocess.run([exe, "-q", "-x", base, "-1", f1, "-2", f2, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
-                           stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, env=dict(os.environ, CFB_TEXT_BLOCK="40000"))
-        assert p.returncode != 0
-        assert b"fewer reads in file specified with -2" in p.stderr
+    r = util.reference_run("class", ["-q", "-x", base, "-1", f1, "-2", f2], str(tmp_path / "ref"))
+    assert r["rc"] != 0 and any("fewer reads in file specified with -2" in l for l in r["errors"]), r
+    p = subprocess.run([EXE, "-q", "-x", base, "-1", f1, "-2", f2, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
+                       stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, env=dict(os.environ, CFB_TEXT_BLOCK="40000"))
+    assert p.returncode != 0
+    assert b"fewer reads in file specified with -2" in p.stderr
 
 
 def test_fasta_record_wrapped_across_a_span_cut(syn, tmp_path):

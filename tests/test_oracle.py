@@ -1,6 +1,8 @@
 """CPU suite: pins the oracle (oracle/cf_oracle.cpp) against the reference's outputs, and the
-product's host-compilable classification logic against the oracle.  No GPU needed."""
+product's host-compilable classification logic against the oracle.  No GPU needed, except where a synthetic
+index comes from the product's builder (marked gpu)."""
 import ctypes as C
+import hashlib
 import lzma
 import os
 import re
@@ -45,13 +47,14 @@ def test_oracle_matches_manual_example(tmp_path):
     """The reference's only known-answer fixture (MANUAL.markdown:1586-1603)."""
     util.ensure_oracle()
     base, reads = util.golden_index("example"), os.path.join(util.GOLDEN, "example.reads.fa")   # committed copy (tests/golden/make_example_golden.py)
-    ex = "/root/reference/example"
-    if os.path.exists(ex):        # where the reference tree is present: the copy is the reference's own bytes
-        for k in "1234":
-            with open("%s/index/test.%s.cf" % (ex, k), "rb") as f, open("%s.%s.cf" % (base, k), "rb") as g:
-                assert f.read() == g.read()
-        with open(ex + "/reads/input.fa", "rb") as f, open(reads, "rb") as g:
-            assert f.read() == g.read()
+    # the copy is the reference's own bytes: sha256 of its example/index/test.{1,2,3,4}.cf and example/reads/input.fa
+    ref_sha256 = {".1.cf": "73894274fbeef3ff3927e50f5d7896693b821b25d84888f2113d019edbc16ad3", ".2.cf": "864df23898e55c42f5a04f23ce85528255dfa0ef51313f9db84ee6e0560e826e",
+                  ".3.cf": "65cf2737ded0050ff8f00947322934b1c987c07b31033ba661072cc4b77df032", ".4.cf": "876eff21a39ac41dbd88421eea70dc9c23474e39b7ff338ab5d500e24dc37364"}
+    for ext, want in ref_sha256.items():
+        with open(base + ext, "rb") as f:
+            assert hashlib.sha256(f.read()).hexdigest() == want, ext
+    with open(reads, "rb") as f:
+        assert hashlib.sha256(f.read()).hexdigest() == "885b4f7483e0814d2ce9b935465735f9dbcd3f8ed7c0eaee363834b87b93bfb9"
     tsv, rep = util.run_cli(util.ORACLE_BIN, ["-f", "-x", base, "-U", reads], str(tmp_path / "o.tsv"), str(tmp_path / "o.rep"))
     with open(os.path.join(util.GOLDEN, "example.tsv"), "rb") as f:
         assert tsv == f.read()
@@ -64,7 +67,7 @@ def test_oracle_matches_manual_example(tmp_path):
     assert all(r[3] == "4225" for r in rows)
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not built")
+@pytest.mark.gpu      # the index comes from the product's builder
 @pytest.mark.parametrize("opts", [[], ["-k", "1"], ["--classification-rank", "genus"], ["--min-hitlen", "30", "-k", "3"]])
 def test_oracle_matches_live_reference_synthetic(opts, tmp_path):
     """Seeded synthetic genus/species index (SURVEY Appendix C recipe, with strains), SE FASTA + PE FASTQ."""
@@ -74,16 +77,16 @@ def test_oracle_matches_live_reference_synthetic(opts, tmp_path):
     rd = util.synth.sample_reads(seqs, 3000, 100, seed=11, lens=(40, 220))
     fa = str(tmp_path / "r.fa")
     util.synth.write_fasta(fa, rd)
-    a = util.run_cli(util.REF_CLASS, ["-f", "-x", base, "-U", fa] + opts, str(tmp_path / "a.tsv"), str(tmp_path / "a.rep"))
+    a = util.reference_cli(["-f", "-x", base, "-U", fa] + opts, tmp_path)
     b = util.run_cli(util.ORACLE_BIN, ["-f", "-x", base, "-U", fa] + opts, str(tmp_path / "b.tsv"), str(tmp_path / "b.rep"))
-    assert a == b
+    assert a == util.digests(b)
     prs = util.synth.sample_pairs(seqs, 1500, 125, seed=12)
     f1, f2 = str(tmp_path / "p_1.fq"), str(tmp_path / "p_2.fq")
     util.synth.write_fastq(f1, [(n, x) for n, x, _ in prs])
     util.synth.write_fastq(f2, [(n, y) for n, _, y in prs], qual=b"5")
-    a = util.run_cli(util.REF_CLASS, ["-q", "-x", base, "-1", f1, "-2", f2] + opts, str(tmp_path / "a.tsv"), str(tmp_path / "a.rep"))
+    a = util.reference_cli(["-q", "-x", base, "-1", f1, "-2", f2] + opts, tmp_path)
     b = util.run_cli(util.ORACLE_BIN, ["-q", "-x", base, "-1", f1, "-2", f2] + opts, str(tmp_path / "b.tsv"), str(tmp_path / "b.rep"))
-    assert a == b
+    assert a == util.digests(b)
 
 
 @pytest.mark.parametrize("case", sorted(PARAM_CASES))
@@ -105,7 +108,7 @@ def test_product_logic_matches_oracle_adversarial(case, adv_base, adv_reads):
     o.close(); h.close()
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="needs oracle/_ref/centrifuge-build-bin to make the fixture")
+@pytest.mark.gpu      # the index comes from the product's builder
 def test_product_logic_matches_oracle_paired_and_wide_sample():
     """> 65535 sequences (u32 SA sample, boundary rows), paired units with filtered mates."""
     import numpy as np
@@ -132,9 +135,7 @@ def test_product_logic_matches_oracle_paired_and_wide_sample():
                 f.write("%d\t|\t%d\t|\tspecies\t|\n" % (1000 + t, 100 + t % 30))
         with open(os.path.join(d, "names.dmp"), "w") as f:
             f.write("1\t|\troot\t|\t\t|\tscientific name\t|\n")
-        subprocess.check_call([util.REF_BUILD, "-p", "4", "--conversion-table", os.path.join(d, "conv.tsv"), "--taxonomy-tree",
-                               os.path.join(d, "nodes.dmp"), "--name-table", os.path.join(d, "names.dmp"), os.path.join(d, "g.fa"), base],
-                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        util.build_fasta_index([os.path.join(d, "g.fa")], os.path.join(d, "conv.tsv"), os.path.join(d, "nodes.dmp"), os.path.join(d, "names.dmp"), base)
     A = util.synth.ACGT
     m1, m2 = [], []
     for k in range(1500):
@@ -216,7 +217,7 @@ def test_product_loader_host_only(adv_base):
     ix.close()
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
+@pytest.mark.gpu      # the index comes from the product's builder
 @pytest.mark.parametrize("kind", ["too_many", "too_few", "space", "control", "plus_one"])
 def test_oracle_reader_rejects_what_the_reference_rejects(kind, tmp_path):
     """FASTQ quality-string rules (pat.cpp:1042-1078): same message and a failing exit status, or the same output."""
@@ -230,12 +231,10 @@ def test_oracle_reader_rejects_what_the_reference_rejects(kind, tmp_path):
             if i == 200:
                 q = {"too_many": q + b"FF", "too_few": q[:-1], "space": q[:10] + b" " + q[11:], "control": q[:10] + b"\x1f" + q[11:], "plus_one": q + b"F"}[kind]
             f.write(b"@" + name.encode() + b"\n" + a.tobytes() + b"\n+\n" + q + b"\n")
-    outs = []
-    for exe in (util.REF_CLASS, util.ORACLE_BIN):
-        p = subprocess.run([exe, "-q", "-x", base, "-U", fq, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
-                           stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
-        msgs = [l for l in p.stderr.decode().splitlines() if l.startswith("Error") or l.startswith("Saw ASCII")]
-        with open(tmp_path / "o.tsv", "rb") as f:
-            outs.append((p.returncode != 0, msgs, f.read() if p.returncode == 0 else b""))
+    r = util.reference_run("class", ["-q", "-x", base, "-U", fq], str(tmp_path))
+    outs = [(r["rc"] != 0, r["errors"], r["outputs"][0] if r["rc"] == 0 else None)]
+    p = subprocess.run([util.ORACLE_BIN, "-q", "-x", base, "-U", fq, "-S", str(tmp_path / "o.tsv"), "--report-file", str(tmp_path / "o.rep")],
+                       stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+    outs.append((p.returncode != 0, util.error_lines(p.stderr), util.file_digest(tmp_path / "o.tsv") if p.returncode == 0 else None))
     assert outs[0] == outs[1]
     assert outs[0][0] == (kind != "plus_one")

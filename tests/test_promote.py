@@ -1,6 +1,6 @@
 """`centrifuge-promote` equivalent (SURVEY.md 8f rank 4): cfb_promote / `centrifuge-class --promote` against the
-reference's own Perl script -- committed goldens (tests/golden/make_promote_golden.py) and, where the script is
-present, differential fuzzing against the live script."""
+reference's own Perl script -- committed goldens (tests/golden/make_promote_golden.py) and differential fuzzing
+against recorded runs of the script (tests/golden/reference_runs.json)."""
 import ctypes as C
 import lzma
 import os
@@ -50,20 +50,11 @@ def test_cli_promote_mode(tmp_path):
         assert p.stdout == g.read()
 
 
-@pytest.mark.skipif(not (os.path.exists("/root/reference/centrifuge-promote") and util.have_ref()), reason="needs the reference's Perl script (build container only)")
 def test_promote_matches_reference_script_on_random_tables(tmp_path):
-    """Differential fuzzing against the live Perl script: taxIDs at every level of the tree and outside it, dotted
+    """Differential fuzzing against recorded runs of the Perl script: taxIDs at every level of the tree and outside it, dotted
     strain IDs, runs of equal read names, repeated names, unclassified rows, every level."""
     import random
-    import shutil
-    import stat
     base = util.golden_index("adv")
-    stage = tmp_path / "stage"
-    stage.mkdir()
-    shutil.copy("/root/reference/centrifuge-promote", stage / "centrifuge-promote")
-    shim = stage / "centrifuge-inspect"
-    shim.write_text("#!/bin/sh\nexec %s \"$@\"\n" % os.path.join(util.REFDIR, "centrifuge-inspect-bin"))
-    shim.chmod(shim.stat().st_mode | stat.S_IEXEC)
     taxa = [0, 1, 10, 11, 100, 101, 102, 103] + list(range(1000, 1020)) + [424242]
     for case in range(60):
         rng = random.Random(77 + case)
@@ -79,7 +70,7 @@ def test_promote_matches_reference_script_on_random_tables(tmp_path):
         tsv = tmp_path / "t.tsv"
         tsv.write_text("\n".join(rows) + ("\n" if rng.random() < 0.9 else ""))
         level = rng.choice(LEVELS + ["order", "no rank"])
-        p = subprocess.run(["perl", str(stage / "centrifuge-promote"), base, str(tsv), level], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL)
+        p = util.reference_run("promote", [base, str(tsv), level])
         out = tmp_path / "o.tsv"
         assert lib().cfb_promote(base.encode(), str(tsv).encode(), level.encode(), str(out).encode()) == 0
-        assert out.read_bytes() == p.stdout, (case, level)
+        assert util.digest(out.read_bytes()) == p["stdout"], (case, level)

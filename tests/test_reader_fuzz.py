@@ -27,20 +27,18 @@ def _case(case, seed0):
     return fasta, (mutate_fasta(rng, sub) if fasta else mutate_fastq(rng, sub)), TRIMS[rng.randrange(len(TRIMS))]
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
 def test_oracle_file_driver_matches_reference_on_irregular_text(tmp_path):
     util.ensure_oracle()
     base = util.golden_index("adv")
 
-    def run(exe, fmt, path, tag, trims):
-        tsv, rep = str(tmp_path / (tag + ".tsv")), str(tmp_path / (tag + ".rep"))
-        p = subprocess.run([exe, fmt, "-x", base, "-U", path, "-S", tsv, "--report-file", rep, "-5", str(trims[0]), "-3", str(trims[1])],
-                           stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
-        msgs = [l for l in p.stderr.decode(errors="replace").splitlines() if l.startswith("Error") or l.startswith("Saw ASCII")]
-        if p.returncode != 0:
-            return ("fail", msgs)
-        with open(tsv, "rb") as f, open(rep, "rb") as g:
-            return ("ok", f.read(), g.read())
+    def run(fmt, path, trims):
+        args = [fmt, "-x", base, "-U", path, "-5", str(trims[0]), "-3", str(trims[1])]
+        r = util.reference_run("class", args, str(tmp_path / "ref"))
+        want = ("fail", r["errors"]) if r["rc"] != 0 else ("ok",) + tuple(r["outputs"])
+        tsv, rep = str(tmp_path / "ora.tsv"), str(tmp_path / "ora.rep")
+        p = subprocess.run([util.ORACLE_BIN] + args + ["-S", tsv, "--report-file", rep], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+        got = ("fail", util.error_lines(p.stderr)) if p.returncode != 0 else ("ok", util.file_digest(tsv), util.file_digest(rep))
+        return want, got
 
     for case in range(N_CASES):
         fasta, data, trims = _case(case, 1000)
@@ -48,10 +46,10 @@ def test_oracle_file_driver_matches_reference_on_irregular_text(tmp_path):
         with open(path, "wb") as f:
             f.write(data)
         fmt = "-f" if fasta else "-q"
-        assert run(util.REF_CLASS, fmt, path, "ref", trims) == run(util.ORACLE_BIN, fmt, path, "ora", trims), (case, fmt, trims)
+        want, got = run(fmt, path, trims)
+        assert want == got, (case, fmt, trims)
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref reference binaries not shipped")
 def test_oracle_file_driver_matches_reference_on_irregular_mate_files(tmp_path):
     """Paired input: independently mutated mate files, including the ones that fall out of step
     ("fewer reads in file specified with -1/-2": same message, failing exit status)."""
@@ -59,14 +57,14 @@ def test_oracle_file_driver_matches_reference_on_irregular_mate_files(tmp_path):
     base = util.golden_index("adv")
     reads = clean_reads()
 
-    def run(exe, fmt, p1, p2, tag):
-        tsv, rep = str(tmp_path / (tag + ".tsv")), str(tmp_path / (tag + ".rep"))
-        p = subprocess.run([exe, fmt, "-x", base, "-1", p1, "-2", p2, "-S", tsv, "--report-file", rep], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
-        msgs = [l for l in p.stderr.decode(errors="replace").splitlines() if l.startswith("Error") or l.startswith("Saw ASCII")]
-        if p.returncode != 0:
-            return ("fail", msgs)
-        with open(tsv, "rb") as f, open(rep, "rb") as g:
-            return ("ok", f.read(), g.read())
+    def run(fmt, p1, p2):
+        args = [fmt, "-x", base, "-1", p1, "-2", p2]
+        r = util.reference_run("class", args, str(tmp_path / "ref"))
+        want = ("fail", r["errors"]) if r["rc"] != 0 else ("ok",) + tuple(r["outputs"])
+        tsv, rep = str(tmp_path / "ora.tsv"), str(tmp_path / "ora.rep")
+        p = subprocess.run([util.ORACLE_BIN] + args + ["-S", tsv, "--report-file", rep], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+        got = ("fail", util.error_lines(p.stderr)) if p.returncode != 0 else ("ok", util.file_digest(tsv), util.file_digest(rep))
+        return want, got
 
     for case in range(100):
         rng = random.Random(424200 + case)
@@ -80,7 +78,8 @@ def test_oracle_file_driver_matches_reference_on_irregular_mate_files(tmp_path):
         with open(p2, "wb") as f:
             f.write(mut(rng, sub2))
         fmt = "-f" if fasta else "-q"
-        assert run(util.REF_CLASS, fmt, p1, p2, "ref") == run(util.ORACLE_BIN, fmt, p1, p2, "ora"), (case, fmt)
+        want, got = run(fmt, p1, p2)
+        assert want == got, (case, fmt)
 
 
 def test_product_reader_matches_oracle_reader_on_irregular_text(tmp_path):

@@ -3,6 +3,7 @@ oracle (oracle/_ref/libcforacle.so, test infrastructure) and of the host-compile
 logic (tests/native/hostlogic.cpp)."""
 import ctypes as C
 import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -31,8 +32,111 @@ for ch, v in (("A", 0), ("C", 1), ("G", 2), ("T", 3), ("N", 4)):
     ASC2DNA[ord(ch.lower())] = v
 
 
-def have_ref():
-    return os.path.exists(REF_CLASS) and os.path.exists(REF_BUILD)
+# ----------------------------------------------------------------------------- recorded reference runs
+# The tests compare with what the unmodified reference did for the same call.  Those results are stored in
+# tests/golden/reference_runs.json, keyed by the tool, its arguments and the contents of every input file and
+# index they name, so the suite needs neither the reference sources nor its binaries.  With CFB_RECORD_REFERENCE
+# set to a file name, every call runs the real binary (oracle/_ref, built from the reference sources by
+# `make -C oracle ref`) and appends its result there; tests/golden/merge_reference_runs.py folds such files in.
+# A test that skips while recording (one that needs two GPUs, say) makes no calls, so its runs are recorded on a
+# machine where it runs, or by making the same calls from a script (the reference's binaries need no GPU).
+REFERENCE_RUNS = os.path.join(GOLDEN, "reference_runs.json")
+RECORD = os.environ.get("CFB_RECORD_REFERENCE")
+_runs = None
+
+
+def digest(data):
+    return hashlib.sha256(data).hexdigest()[:32]
+
+
+def file_digest(path):
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for blk in iter(lambda: f.read(1 << 24), b""):
+            h.update(blk)
+    return h.hexdigest()[:32]
+
+
+def _key_token(arg):
+    """An argument as it enters the key: input files and index bases by content, other words as they are."""
+    parts = []
+    for p in str(arg).split(","):
+        if os.path.isfile(p):
+            parts.append("file:" + file_digest(p))
+        elif os.path.isfile(p + ".1.cf"):
+            parts.append("index:" + "".join(file_digest("%s.%s.cf" % (p, k)) for k in "1234"))
+        else:
+            assert not os.path.isabs(p), "reference call names a path that does not exist: %s" % p
+            parts.append(p)
+    return ",".join(parts)
+
+
+def error_lines(stderr):
+    return [l for l in stderr.decode(errors="replace").splitlines() if l.startswith("Error") or l.startswith("Saw ASCII")]
+
+
+def reference_run(tool, args, out=None):
+    """What the reference's `tool` ("class", "build", "kreport" or "promote") did when run with `args`:
+    dict(rc=exit status, errors=its 'Error' / 'Saw ASCII' lines on stderr, outputs=digests of what it wrote, None
+    where it wrote nothing) and, for the Perl scripts, whose result is what they print, stdout=digest of stdout.  `out` (not part of the key): for "class" a directory for the
+    TSV and report (-S / --report-file), for "build" the index base the .1-.4.cf files go to."""
+    global _runs
+    key = digest(json.dumps([tool] + [_key_token(a) for a in args]).encode())
+    if RECORD:
+        res = _run_reference(tool, list(args), out)
+        with open(RECORD, "a") as f:
+            f.write(json.dumps({key: res}) + "\n")
+        return res
+    if _runs is None:
+        with open(REFERENCE_RUNS) as f:
+            _runs = json.load(f)
+    if key not in _runs:
+        raise KeyError("no recorded reference run for %s %s: record one with CFB_RECORD_REFERENCE (tests/util.py)" % (tool, list(args)))
+    return _runs[key]
+
+
+def _run_reference(tool, args, out):
+    """Runs the reference binary; what the binaries print on stdout (paths, timings) is not part of the result."""
+    if tool in ("kreport", "promote"):
+        return _run_reference_script(tool, args)
+    if tool == "class":
+        os.makedirs(out, exist_ok=True)
+        outputs = [os.path.join(out, "ref.tsv"), os.path.join(out, "ref.rep")]
+        cmd = [REF_CLASS] + args + ["-S", outputs[0], "--report-file", outputs[1]]
+    else:
+        outputs = ["%s.%s.cf" % (out, k) for k in "1234"]
+        cmd = [REF_BUILD] + args + [out]
+    for o in outputs:
+        if os.path.exists(o):
+            os.remove(o)
+    p = subprocess.run(cmd, stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+    return dict(rc=p.returncode, errors=error_lines(p.stderr), outputs=[file_digest(o) if os.path.exists(o) else None for o in outputs])
+
+
+def _run_reference_script(tool, args):
+    import shutil
+    import stat
+    with tempfile.TemporaryDirectory() as stage:      # the Perl scripts look for centrifuge-inspect beside themselves
+        script = os.path.join(stage, "centrifuge-" + tool)
+        shutil.copy(os.path.join(os.environ["CFB_REFERENCE_SRC"], "centrifuge-" + tool), script)
+        shim = os.path.join(stage, "centrifuge-inspect")
+        with open(shim, "w") as f:
+            f.write("#!/bin/sh\nexec %s \"$@\"\n" % os.path.join(REFDIR, "centrifuge-inspect-bin"))
+        os.chmod(shim, os.stat(shim).st_mode | stat.S_IEXEC)
+        p = subprocess.run(["perl", script] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+    return dict(rc=p.returncode, errors=error_lines(p.stderr), stdout=digest(p.stdout), outputs=[])
+
+
+def reference_cli(args, tmp):
+    """Digests of the classification TSV and report the reference's centrifuge-class writes for `args`
+    (it must succeed); compare with `digests(run_cli(...))`."""
+    r = reference_run("class", args, os.path.join(str(tmp), "reference"))
+    assert r["rc"] == 0, r
+    return tuple(r["outputs"])
+
+
+def digests(outputs):
+    return tuple(digest(x) for x in outputs)
 
 
 def ensure_oracle():
@@ -50,20 +154,31 @@ def ensure_oracle():
 
 
 # ----------------------------------------------------------------------------- fixtures
-def build_index(tag, genera, species, length, seed, div=0.03, cid=False, strains=False, extra_args=()):
-    """Synthetic genomes -> .cf index through the reference's own builder (oracle/_ref).  Cached."""
-    key = hashlib.md5(repr((tag, genera, species, length, seed, div, cid, strains, extra_args)).encode()).hexdigest()[:12]
+def build_index(tag, genera, species, length, seed, div=0.03, cid=False, strains=False):
+    """Synthetic genomes -> .cf index through the product's builder (needs a GPU), checked against the reference's
+    centrifuge-build-bin on the same files.  Cached."""
+    key = hashlib.md5(repr((tag, genera, species, length, seed, div, cid, strains, ())).encode()).hexdigest()[:12]
     d = os.path.join(CACHE, "%s_%s" % (tag, key))
     base = os.path.join(d, "idx")
     if not os.path.exists(base + ".4.cf"):
-        if not have_ref():
-            raise RuntimeError("oracle/_ref/centrifuge-build-bin missing (run `make -C oracle ref` where /root/reference exists)")
         os.makedirs(d, exist_ok=True)
         synth.write_genomes(d, genera, species, length, seed, div, cid, strains)
-        with open(os.path.join(d, "build.log"), "w") as log:
-            subprocess.check_call([REF_BUILD, "-p", "4", "--conversion-table", os.path.join(d, "conv.tsv"),
-                                   "--taxonomy-tree", os.path.join(d, "nodes.dmp"), "--name-table", os.path.join(d, "names.dmp")]
-                                  + list(extra_args) + [os.path.join(d, "genomes.fa"), base], stdout=log, stderr=log)
+        build_fasta_index([os.path.join(d, "genomes.fa")], os.path.join(d, "conv.tsv"), os.path.join(d, "nodes.dmp"), os.path.join(d, "names.dmp"), base)
+    return base
+
+
+def build_fasta_index(fasta, conv, nodes, names, base):
+    """cfb_build_index over FASTA files; the .1-.4.cf files must be the bytes centrifuge-build-bin -p 4 writes
+    (recorded reference run), else they are removed and the call fails."""
+    from centrifuge_b200 import capi
+    want = reference_run("build", ["-p", "4", "--conversion-table", conv, "--taxonomy-tree", nodes, "--name-table", names, ",".join(fasta)], base + "_reference")
+    capi.build_index(capi.build_opts(base, fasta=list(fasta), conversion_table=conv, taxonomy_tree=nodes, name_table=names))
+    files = ["%s.%s.cf" % (base, k) for k in "1234"]
+    bad = [f for f, w in zip(files, want["outputs"]) if file_digest(f) != w]
+    if bad:
+        for f in files:
+            os.remove(f)
+        raise AssertionError("the product's builder does not write the reference's bytes: %s" % ", ".join(os.path.basename(f) for f in bad))
     return base
 
 
